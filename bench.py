@@ -324,11 +324,13 @@ def measure(name, B, steps, warmup, rank, world, local, dev, dist, want_e2e=True
     x_host = (torch.rand(B, 3, S, S, generator=g) * 2 - 1).pin_memory()
     x_dev = x_host.to(dev)
     gathered = [torch.empty_like(x_dev) for _ in range(world)] if world > 1 else None
+    last = {}
 
     def one_step(seed):
         out = eng.purify(x_dev, cond, coef, sx, se, update_kind=update_kind, seed=seed, sample_offset=rank * B)
         if world > 1:
             dist.all_gather(gathered, out)
+        last["purified"] = out
         return out
 
     def timed(fn, k):
@@ -357,6 +359,8 @@ def measure(name, B, steps, warmup, rank, world, local, dev, dist, want_e2e=True
     ms_total = timed(one_step, steps)
     clocks = sampler.stop() if sampler else None
     value = world * B * steps / (ms_total / 1e3)
+    # the images the last timed step returned (every rank's, in rank order), before the runs below reuse the engine
+    purified = (torch.cat(gathered) if world > 1 else last["purified"]).float().cpu()
 
     # ---- e2e through the runner API from pinned host memory ----------------------------------------------
     e2e = None
@@ -382,7 +386,7 @@ def measure(name, B, steps, warmup, rank, world, local, dev, dist, want_e2e=True
                "api": f"{R.__module__}.{R.__name__}.image_editing_sample"}
 
     res = {"value": value, "ms_per_step": ms_total / steps, "clocks": clocks, "e2e": e2e, "nsteps": nsteps,
-           "launches": steps * (nsteps * eng.launches_per_step + 2), "B": B}
+           "launches": steps * (nsteps * eng.launches_per_step + 2), "B": B, "purified": purified}
     if rank == 0:
         res["roofline"] = roofline_of(eng, wl, B, value / world, nsteps)
     res["engine"] = eng
@@ -431,6 +435,21 @@ def roofline_of(eng, wl, B, value_per_gpu, nsteps):
     return roofline
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, purified):
+    """Save what the timed path returned so that two builds run with the same arguments (same seeded weights, images
+    and noise) can be compared output for output. Above DUMP_LIMIT, a seeded sample of whole images is kept."""
+    n = purified.shape[0]
+    keep = max(1, DUMP_LIMIT // (purified[0].numel() * 4))
+    if keep < n:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        purified = purified[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "purified.npy"), purified.numpy().astype(np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -443,7 +462,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the embedded ADM (configs[2]) measurement")
     ap.add_argument("--no-gpu-eager", action="store_true", help="skip the same-GPU PyTorch-eager baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the images the last timed step returned to DIR/purified.npy (float32; at most "
+                         f"{DUMP_LIMIT >> 20} MB: beyond that a fixed, seeded sample of whole images in batch order)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -464,6 +488,9 @@ def main():
     steps, warmup = args.steps, args.warmup
     main_res = measure(args.config, B, steps, warmup, rank, world, local, dev, dist, want_e2e=not args.no_e2e)
     main_res.pop("engine").close()
+    purified = main_res.pop("purified")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, purified)
 
     secondary = None
     if args.config == "cifar10" and world == 1 and not args.no_secondary:

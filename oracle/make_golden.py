@@ -164,7 +164,8 @@ def golden_adm_and_celeba():
     print("celeba tiny |y|", y.abs().mean().item())
 
 
-if __name__ == "__main__" and not ({"--siblings", "--adm-vpsde", "--checkpoint-keys", "--guided-schedules"} & set(sys.argv)):
+if __name__ == "__main__" and not ({"--siblings", "--adm-vpsde", "--checkpoint-keys", "--guided-schedules",
+                                    "--reference-interfaces"} & set(sys.argv)):
     if "--adm-celeba" not in sys.argv:
         main()
     if "--ncsnpp" not in sys.argv:
@@ -328,3 +329,160 @@ def golden_guided_schedules():
 
 if __name__ == "__main__" and "--guided-schedules" in sys.argv:
     golden_guided_schedules()
+
+
+def golden_reference_interfaces():
+    """What four CPU tests compare against, recorded from the reference so that they need only the repository:
+      reference_checkpoints.npz   two score_sde checkpoints (plain and DataParallel 'module.' keys) written by the
+                                  reference's own NCSNpp + optimizer + ExponentialMovingAverage, and the state dict its
+                                  restore_checkpoint + ema.copy_to produce from them (runners/diffpure_sde.py:42-47,178-182)
+      reference_interfaces.json   the state_dict() names / shapes / dtypes of the reduced ADM (after convert_to_fp16) and
+                                  CelebA modules with the configs that built them; the runner classes eval_sde_adv.py
+                                  imports and the calls its SDE_Adv_Model (L34-93) makes on them, with configs/cifar10.yml
+      spaced_timesteps.npz        guided_diffusion/respace.py:space_timesteps on seeded random section specs, every 'ddimN'
+                                  of a 300-step chain, and the specs it rejects"""
+    import contextlib
+    import io
+    import json
+    import tempfile
+    import types
+    from types import SimpleNamespace as NS
+    torch.set_grad_enabled(False)
+    ref_import.install()
+
+    # ---- checkpoints through the reference's loader -------------------------------------------------------------
+    from score_sde.models.ema import ExponentialMovingAverage
+    from score_sde.losses import get_optimizer
+    from runners.diffpure_sde import restore_checkpoint
+    over = dict(nf=8, ch_mult=[1, 2], num_res_blocks=1, attn_resolutions=[8], **{"data.image_size": 16})
+    ck, want = {}, None
+    for wrap in (False, True):
+        model, cfg = ref_import.build_ncsnpp(over)
+        if wrap:
+            model = torch.nn.DataParallel(model)
+        for i, p in enumerate(model.parameters()):   # every tensor distinct (offset i) and varying inside (a period-7
+            p.data.copy_(i + (torch.arange(p.numel()) % 7 - 3).reshape(p.shape) / 8)  # ramp): exposes ordering mistakes
+        ema = ExponentialMovingAverage(model.parameters(), decay=0.5)
+        for p in model.parameters():                 # the weights move away from the EMA shadow
+            p.data.add_(0.5)
+        opt = get_optimizer(cfg, model.parameters())
+        with tempfile.TemporaryDirectory() as tmp:
+            path = os.path.join(tmp, "checkpoint_8.pth")
+            torch.save({"optimizer": opt.state_dict(), "model": model.state_dict(), "ema": ema.state_dict(), "step": 3},
+                       path)
+            with open(path, "rb") as f:
+                ck["wrapped" if wrap else "plain"] = np.frombuffer(f.read(), dtype=np.uint8)
+            model2, cfg2 = ref_import.build_ncsnpp(over)
+            if wrap:
+                model2 = torch.nn.DataParallel(model2)
+            ema2 = ExponentialMovingAverage(model2.parameters(), decay=cfg2.model.ema_rate)
+            state = dict(step=0, optimizer=get_optimizer(cfg2, model2.parameters()), model=model2, ema=ema2)
+            restore_checkpoint(path, state, "cpu")
+            ema2.copy_to(model2.parameters())
+        got = (model2.module if wrap else model2).state_dict()
+        if want is None:
+            want = got
+        assert list(got) == list(want) and all(torch.equal(got[k], want[k]) for k in want)
+    buf = io.BytesIO()
+    torch.save(want, buf)
+    np.savez_compressed(os.path.join(OUT, "reference_checkpoints.npz"), ckpt_plain=ck["plain"], ckpt_wrapped=ck["wrapped"],
+                        want=np.frombuffer(buf.getvalue(), dtype=np.uint8))
+    print("checkpoints:", len(want), "tensors,", {k: v.size for k, v in ck.items()}, "bytes")
+
+    # ---- module state dicts and the configs behind them ------------------------------------------------------------
+    def listing(sd):
+        return [[k, list(v.shape), str(v.dtype).replace("torch.", "")] for k, v in sd.items()]
+
+    def plain(ns):
+        return {k: plain(v) for k, v in vars(ns).items()} if isinstance(ns, NS) else ns
+
+    out = {}
+    m, _, mc = ref_import.build_adm(num_channels=64, image_size=64, num_res_blocks=1, use_fp16=True)
+    out["adm"] = {"model_config": dict(mc), "state_dict": listing(m.state_dict())}
+    mc_, ccfg = ref_import.build_celeba({"ch": 64, "ch_mult": [1, 2, 2], "num_res_blocks": 1, "attn_resolutions": [16],
+                                        "data.image_size": 32})
+    out["celeba"] = {"config": plain(ccfg), "state_dict": listing(mc_.state_dict())}
+
+    # ---- eval_sde_adv.SDE_Adv_Model on a recording stand-in for the runners package ---------------------------------
+    rec = {"imports": {}, "constructions": []}
+    args = NS(classifier_name="x", domain="cifar10", t=5, rand_t=False, t_delta=15, use_bm=False, score_type="score_sde",
+              sample_step=1, log_dir="unused", verbose=False)
+    config = ref_import.load_config("cifar10.yml")
+    cifar10_yml = plain(config)
+    config.device = torch.device("cpu")
+    names = {id(args): "args", id(config): "config", id(config.device): "config.device"}
+
+    def recording_module(modname):
+        mod = types.ModuleType(modname)
+
+        def getattr_(cls_name):
+            if cls_name.startswith("__"):                # the import system's own probes (__path__, ...)
+                raise AttributeError(cls_name)
+            if cls_name not in rec["imports"].setdefault(modname, []):
+                rec["imports"][modname].append(cls_name)
+
+            class Runner:
+                def __init__(self, *a, **kw):
+                    rec["constructions"].append({"diffusion_type": args.diffusion_type, "module": modname,
+                                                 "class": cls_name, "args": [names[id(v)] for v in a],
+                                                 "kwargs": {k: names[id(v)] for k, v in kw.items()}})
+            return Runner
+        mod.__getattr__ = getattr_
+        return mod
+
+    saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "runners" or k.startswith("runners.")}
+    try:
+        sys.modules["runners"] = types.ModuleType("runners")
+        for sub in ("diffpure_ddpm", "diffpure_guided", "diffpure_sde", "diffpure_ode", "diffpure_ldsde"):
+            sys.modules["runners." + sub] = recording_module("runners." + sub)
+        sys.modules.pop("eval_sde_adv", None)
+        import eval_sde_adv
+        eval_sde_adv.get_image_classifier = lambda name: torch.nn.Identity()
+        for dt in ("ddpm", "sde", "ode", "ldsde", "celebahq-ddpm"):
+            args.diffusion_type = dt
+            with contextlib.redirect_stdout(io.StringIO()):
+                eval_sde_adv.SDE_Adv_Model(args, config)
+    finally:
+        for k in [k for k in sys.modules if k == "runners" or k.startswith("runners.") or k == "eval_sde_adv"]:
+            sys.modules.pop(k)
+        sys.modules.update(saved)
+    out["sde_adv_model"] = dict(rec, cifar10_yml=cifar10_yml)
+    with open(os.path.join(OUT, "reference_interfaces.json"), "w") as f:
+        json.dump(out, f)
+    print("interfaces:", len(out["adm"]["state_dict"]), "ADM tensors,", len(out["celeba"]["state_dict"]),
+          "CelebA tensors,", len(rec["constructions"]), "runner constructions")
+
+    # ---- respace.space_timesteps -------------------------------------------------------------------------------------
+    from guided_diffusion.respace import space_timesteps
+    rng = np.random.default_rng(7)
+    rn, rspec, rkept = [], [], []
+    for _ in range(300):
+        n = int(rng.integers(8, 1200))
+        k = int(rng.integers(1, 6))
+        size = n // k
+        counts = [int(rng.integers(1, max(2, min(size, 60)))) for _ in range(k)]
+        rn.append(n)
+        rspec.append(",".join(str(c) for c in counts))
+        rkept.append(sorted(space_timesteps(n, rspec[-1])))
+    dn, dkept, rejected = [], [], []
+    for want_n in range(1, 301):
+        try:
+            dkept.append(sorted(space_timesteps(300, f"ddim{want_n}")))
+            dn.append(want_n)
+        except ValueError:
+            rejected.append((300, f"ddim{want_n}"))
+    for bad in ("400", "10,200"):
+        try:
+            space_timesteps(300, bad)
+        except ValueError:
+            rejected.append((300, bad))
+    np.savez_compressed(os.path.join(OUT, "spaced_timesteps.npz"), random_n=np.array(rn), random_spec=np.array(rspec),
+                        random_len=np.array([len(v) for v in rkept]), random_kept=np.concatenate(rkept).astype(np.int16),
+                        ddim_n=np.array(dn), ddim_len=np.array([len(v) for v in dkept]),
+                        ddim_kept=np.concatenate(dkept).astype(np.int16),
+                        rejected_n=np.array([r[0] for r in rejected]), rejected_spec=np.array([r[1] for r in rejected]))
+    print("spaced timesteps:", len(rn), "random specs,", len(dn), "feasible ddimN,", len(rejected), "rejected specs")
+
+
+if __name__ == "__main__" and "--reference-interfaces" in sys.argv:
+    golden_reference_interfaces()

@@ -168,33 +168,21 @@ def test_respaced_guided_chains_match_reference_golden():
         schedule.guided_tables(51, 1000, "cosine", "ddim50")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/guided_diffusion"), reason="reference tree not present")
 def test_spaced_timesteps_equals_the_reference_on_random_specs():
     """schedule.spaced_timesteps / oracle _kept_steps vs the reference's own space_timesteps (respace.py:7-60) on seeded random
-    section specs and every feasible 'ddimN' of a 300-step chain; infeasible specs raise ValueError in all three."""
-    from oracle import ref_import
-    ref_import.install()
-    from guided_diffusion.respace import space_timesteps
-    rng = np.random.default_rng(7)
-    for _ in range(300):
-        n = int(rng.integers(8, 1200))
-        k = int(rng.integers(1, 6))
-        size = n // k
-        counts = [int(rng.integers(1, max(2, min(size, 60)))) for _ in range(k)]
-        spec = ",".join(str(c) for c in counts)
-        want = sorted(space_timesteps(n, spec))
-        assert schedule.spaced_timesteps(n, spec) == want == OL._kept_steps(n, spec), (n, spec)
-    for want_n in range(1, 301):
-        try:
-            want = sorted(space_timesteps(300, f"ddim{want_n}"))
-        except ValueError:
+    section specs and every feasible 'ddimN' of a 300-step chain; infeasible specs raise ValueError in all three. The
+    reference's answers are recorded in spaced_timesteps.npz (oracle/make_golden.py --reference-interfaces)."""
+    d = np.load(os.path.join(G, "spaced_timesteps.npz"))
+    rejected = [str(s) for s in d["rejected_spec"]]
+    assert len(d["random_n"]) == 300 and len(d["ddim_n"]) + sum(s.startswith("ddim") for s in rejected) == 300
+    assert {"400", "10,200"} <= set(rejected)
+    for key, specs in (("random", d["random_spec"]), ("ddim", [f"ddim{k}" for k in d["ddim_n"]])):
+        ns = d["random_n"] if key == "random" else [300] * len(specs)
+        kept = np.split(d[key + "_kept"], np.cumsum(d[key + "_len"])[:-1])
+        for n, spec, want in zip(ns, specs, kept):
+            n, spec, want = int(n), str(spec), want.tolist()
+            assert schedule.spaced_timesteps(n, spec) == want == OL._kept_steps(n, spec), (n, spec)
+    for n, bad in zip(d["rejected_n"], d["rejected_spec"]):
+        for fn in (schedule.spaced_timesteps, OL._kept_steps):
             with pytest.raises(ValueError):
-                schedule.spaced_timesteps(300, f"ddim{want_n}")
-            with pytest.raises(ValueError):
-                OL._kept_steps(300, f"ddim{want_n}")
-            continue
-        assert schedule.spaced_timesteps(300, f"ddim{want_n}") == want == OL._kept_steps(300, f"ddim{want_n}")
-    for bad in ("400", "10,200"):
-        for fn in (lambda: space_timesteps(300, bad), lambda: schedule.spaced_timesteps(300, bad), lambda: OL._kept_steps(300, bad)):
-            with pytest.raises(ValueError):
-                fn()
+                fn(int(n), str(bad))

@@ -1,12 +1,16 @@
 """CPU: checkpoint ingest (SURVEY.md section 8f-3). The score_sde checkpoint layout -- DataParallel 'module.' keys, the
 'sigmas' buffer, EMA shadow parameters that replace the weights -- is loaded by diffpure_b200 exactly as the reference's
 restore_checkpoint + ExponentialMovingAverage.copy_to do (runners/diffpure_sde.py:42-47,175-182; score_sde/models/ema.py:61-72)."""
+import io
+import json
 import os
+from types import SimpleNamespace as NS
 
+import numpy as np
 import pytest
 import torch
 
-REF = os.path.isdir("/root/reference/score_sde")
+G = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def _fake_checkpoint(tmp_path):
@@ -34,39 +38,15 @@ def test_score_sde_checkpoint_layout(tmp_path):
         assert torch.equal(sd[k], v), k                  # EMA shadow replaced every weight, in parameter order
 
 
-@pytest.mark.skipif(not REF, reason="reference tree not present")
 @pytest.mark.parametrize("wrap", [False, True])
 def test_score_sde_checkpoint_matches_reference_loader(tmp_path, wrap):
-    """Same file through the reference's own classes (NCSNpp + DataParallel + optimizer + EMA) and through ours."""
-    from oracle import ref_import
-    ref_import.install()
-    over = dict(nf=64, ch_mult=[1, 2], num_res_blocks=1, attn_resolutions=[8], **{"data.image_size": 16})
-    model, cfg = ref_import.build_ncsnpp(over)
-    if wrap:                                              # checkpoints written from a DataParallel model carry 'module.' keys
-        model = torch.nn.DataParallel(model)
-    from score_sde.models.ema import ExponentialMovingAverage
-    from score_sde.losses import get_optimizer
-    from runners.diffpure_sde import restore_checkpoint
-    torch.manual_seed(0)
-    for p in model.parameters():                          # zero-initialised tensors would hide ordering mistakes
-        p.data.normal_()
-    ema = ExponentialMovingAverage(model.parameters(), decay=0.5)
-    for p in model.parameters():
-        p.data.add_(torch.randn_like(p))
-    ema.update(model.parameters())                        # shadow != weights
-    opt = get_optimizer(cfg, model.parameters())
+    """A file written by the reference's own classes (NCSNpp + DataParallel + optimizer + EMA) through ours, against what
+    the reference's restore_checkpoint + ema.copy_to make of it (golden: oracle/make_golden.py --reference-interfaces)."""
+    d = np.load(os.path.join(G, "reference_checkpoints.npz"))
     path = os.path.join(str(tmp_path), "checkpoint_8.pth")
-    torch.save({"optimizer": opt.state_dict(), "model": model.state_dict(), "ema": ema.state_dict(), "step": 3}, path)
-
-    model2, cfg2 = ref_import.build_ncsnpp(over)
-    if wrap:
-        model2 = torch.nn.DataParallel(model2)
-    ema2 = ExponentialMovingAverage(model2.parameters(), decay=cfg2.model.ema_rate)
-    state = dict(step=0, optimizer=get_optimizer(cfg2, model2.parameters()), model=model2, ema=ema2)
-    restore_checkpoint(path, state, "cpu")                # runners/diffpure_sde.py:42-47
-    ema2.copy_to(model2.parameters())                     # L182
-    want = (model2.module if wrap else model2).state_dict()
-
+    with open(path, "wb") as f:
+        f.write(d["ckpt_wrapped" if wrap else "ckpt_plain"].tobytes())
+    want = torch.load(io.BytesIO(d["want"].tobytes()))
     from diffpure_b200.runners.diffpure_sde import _load_score_sde_state
     got = _load_score_sde_state(path)
     assert set(got) == set(want)
@@ -114,41 +94,38 @@ def test_real_checkpoint_key_sets():
     assert {k: tuple(v) for k, v in got.items()} == ck
 
 
-@pytest.mark.skipif(not REF, reason="reference tree not present")
 def test_reference_module_state_dicts_load_directly():
     """state_dict() of the reference's own (reduced) ADM -- after convert_to_fp16, as GuidedDiffusion holds it
     (diffpure_guided.py:31-35) -- and CelebA modules go straight into the runners: names, shapes and dtypes are accepted
-    and the lowered programs reproduce the reference modules through the CPU interpreter."""
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
-    from oracle import ref_import
+    and the lowered programs reproduce the reference modules through the CPU interpreter. The modules' state-dict listings
+    and configs are recorded from the reference (golden: oracle/make_golden.py --reference-interfaces); their outputs for
+    the seeded factory weights are adm_tiny.npz (fp16 torso) and celeba_tiny.npz."""
     from program_interp import Interp
     from diffpure_b200 import lowering_adm as LA, lowering_ddpm as LD
-    from types import SimpleNamespace as NS
-    torch.manual_seed(0)
-    m, _, mc = ref_import.build_adm(num_channels=64, image_size=64, num_res_blocks=1, use_fp16=True)
-    with torch.no_grad():
-        for p_ in m.parameters():                            # zero-initialised layers would make the check vacuous
-            if p_.abs().max() == 0:
-                p_.copy_((torch.randn_like(p_.float()) * 0.02).to(p_.dtype))
-    sd = m.state_dict()
-    assert any(v.dtype == torch.float16 for v in sd.values())
-    cfg = LA.cfg_from_reference(NS(model=NS(**mc)))
-    assert set(LA.param_shapes(cfg)) == set(sd)
-    x = torch.rand(1, 3, 64, 64) * 2 - 1
-    t = torch.tensor([17])
-    with torch.no_grad():
-        y = m(x, t).float()
+    from oracle import adm as A, ddpm_unet as D, weights
+    with open(os.path.join(G, "reference_interfaces.json")) as f:
+        rec = json.load(f)
+    ns = lambda d: json.loads(json.dumps(d), object_hook=lambda o: NS(**o))  # noqa: E731
+
+    def rel(a, b):
+        return ((a - b).norm() / b.norm()).item()
+
+    listing = rec["adm"]["state_dict"]
+    assert any(dt == "float16" for _, _, dt in listing)
+    cfg = LA.cfg_from_reference(ns({"model": rec["adm"]["model_config"]}))
+    assert {k: tuple(v) for k, v in LA.param_shapes(cfg).items()} == {k: tuple(s) for k, s, _ in listing}
+    d = np.load(os.path.join(G, "adm_tiny.npz"))
+    factory = weights.make_state_dict(A.param_shapes(A.tiny_cfg(64, 64, (1, 2, 3, 4), 1, (32, 16, 8))), seed=int(d["seed"]))
+    sd = {k: factory[k].to(getattr(torch, dt)) for k, _, dt in listing}     # the dtypes the reference module holds
     sd32 = {k: v.float() for k, v in sd.items()}
-    got = Interp(LA.lower(cfg, sd32, 1), emulate_bf16=False).run(x, t.float())
-    assert ((got - y).norm() / y.norm()).item() < 2e-2       # the reference ran its torso in fp16
-    mc_, ccfg = ref_import.build_celeba({"ch": 64, "ch_mult": [1, 2, 2], "num_res_blocks": 1, "attn_resolutions": [16],
-                                         "data.image_size": 32})
-    sdc = mc_.state_dict()
-    lcfg = LD.cfg_from_reference(ccfg)
-    assert set(LD.param_shapes(lcfg)) == set(sdc)
-    xc = torch.rand(1, 3, 32, 32) * 2 - 1
-    with torch.no_grad():
-        yc = mc_(xc, torch.tensor([9]))
-    gotc = Interp(LD.lower(lcfg, sdc, 1), emulate_bf16=False).run(xc, torch.tensor([9.0]))
-    assert ((gotc - yc).norm() / yc.norm()).item() < 1e-4
+    got = Interp(LA.lower(cfg, sd32, 2), emulate_bf16=False).run(torch.from_numpy(d["x"]), torch.from_numpy(d["t"]).float())
+    assert rel(got, torch.from_numpy(d["y_fp16"])) < 2e-2                # the reference ran its torso in fp16
+
+    listing = rec["celeba"]["state_dict"]
+    lcfg = LD.cfg_from_reference(ns(rec["celeba"]["config"]))
+    assert {k: tuple(v) for k, v in LD.param_shapes(lcfg).items()} == {k: tuple(s) for k, s, _ in listing}
+    d = np.load(os.path.join(G, "celeba_tiny.npz"))
+    factory = weights.make_state_dict(D.param_shapes(D.tiny_cfg(32, 64, (1, 2, 2), 1, (16,))), seed=int(d["seed"]))
+    sdc = {k: factory[k].to(getattr(torch, dt)) for k, _, dt in listing}
+    gotc = Interp(LD.lower(lcfg, sdc, 2), emulate_bf16=False).run(torch.from_numpy(d["x"]), torch.from_numpy(d["t"]).float())
+    assert rel(gotc, torch.from_numpy(d["y"])) < 1e-4

@@ -1,8 +1,6 @@
 """CPU: ODE / LDSDE sibling loops -- oracle integrands vs the reference's VPODE / LDSDE (golden), schedules vs oracle loops,
 and the drop-in: the reference's unmodified eval_sde_adv.SDE_Adv_Model constructed on top of diffpure_b200.runners."""
 import os
-import sys
-import types
 from types import SimpleNamespace
 
 import numpy as np
@@ -51,44 +49,42 @@ def test_sibling_schedules_reproduce_oracle_loops():
     assert (ref - x).abs().max().item() < 1e-5
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/runners"), reason="reference tree not present")
 def test_reference_sde_adv_model_is_a_drop_in():
-    """The reference's own SDE_Adv_Model (eval_sde_adv.py:34-93), unmodified, on top of this package's runners."""
-    from oracle import ref_import
-    ref_import.install()
-    import diffpure_b200.runners as R
+    """What the reference's own SDE_Adv_Model (eval_sde_adv.py:34-93) asks of its runners, asked of this package's: the
+    runner classes it imports and the constructor calls it makes for each diffusion_type, recorded from the reference with
+    configs/cifar10.yml (golden: oracle/make_golden.py --reference-interfaces), replayed on diffpure_b200.runners."""
+    import importlib
+    import inspect
+    import json
     import diffpure_b200.runners.diffpure_sde as rs
-    import diffpure_b200.runners.diffpure_ode, diffpure_b200.runners.diffpure_ldsde  # noqa: F401,E401
-    import diffpure_b200.runners.diffpure_guided, diffpure_b200.runners.diffpure_ddpm  # noqa: F401,E401
-    saved = {k: sys.modules.get(k) for k in list(sys.modules) if k == "runners" or k.startswith("runners.")}
+    with open(os.path.join(G, "reference_interfaces.json")) as f:
+        rec = json.load(f)["sde_adv_model"]
+    runners = lambda mod: importlib.import_module("diffpure_b200." + mod)  # noqa: E731  ('runners.x' -> ours)
+    assert len(rec["imports"]) == 5
+    for mod, names in rec["imports"].items():
+        for name in names:
+            assert hasattr(runners(mod), name), (mod, name)
+    assert sorted(c["diffusion_type"] for c in rec["constructions"]) == ["celebahq-ddpm", "ddpm", "ldsde", "ode", "sde"]
+    for c in rec["constructions"]:
+        inspect.signature(getattr(runners(c["module"]), c["class"])).bind(*c["args"], **c["kwargs"])
+
+    c = next(c for c in rec["constructions"] if c["diffusion_type"] == "sde")
+    cfg = O.tiny_cfg(64, (1, 2, 2), 1, (16,), 32)
+    sd = weights.make_state_dict(O.param_shapes(cfg), seed=1)
+    args = SimpleNamespace(classifier_name="x", diffusion_type="sde", domain="cifar10", t=5, rand_t=False,
+                           t_delta=15, use_bm=False, score_type="score_sde", sample_step=1, log_dir="/tmp/dp_dropin",
+                           verbose=False)
+    config = json.loads(json.dumps(rec["cifar10_yml"]), object_hook=lambda o: SimpleNamespace(**o))
+    config.model.nf, config.model.ch_mult, config.model.num_res_blocks = 64, [1, 2, 2], 1
+    config.model.attn_resolutions = [16]
+    config.device = torch.device("cpu")
+    value = {"args": args, "config": config, "config.device": config.device}
+    rs_load = rs._load_score_sde_state
+    rs._load_score_sde_state = lambda path, device="cpu": sd
     try:
-        for k in saved:
-            sys.modules.pop(k, None)
-        sys.modules["runners"] = R
-        for sub in ("diffpure_sde", "diffpure_ode", "diffpure_ldsde", "diffpure_guided", "diffpure_ddpm"):
-            sys.modules["runners." + sub] = getattr(R, sub)
-        sys.modules.pop("eval_sde_adv", None)
-        import eval_sde_adv
-        cfg = O.tiny_cfg(64, (1, 2, 2), 1, (16,), 32)
-        sd = weights.make_state_dict(O.param_shapes(cfg), seed=1)
-        rs_load = rs._load_score_sde_state
-        rs._load_score_sde_state = lambda path, device="cpu": sd
-        eval_sde_adv.get_image_classifier = lambda name: torch.nn.Identity()
-        args = SimpleNamespace(classifier_name="x", diffusion_type="sde", domain="cifar10", t=5, rand_t=False,
-                               t_delta=15, use_bm=False, score_type="score_sde", sample_step=1, log_dir="/tmp/dp_dropin",
-                               verbose=False)
-        config = ref_import.load_config("cifar10.yml")
-        config.model.nf, config.model.ch_mult, config.model.num_res_blocks = 64, [1, 2, 2], 1
-        config.model.attn_resolutions = [16]
-        config.device = torch.device("cpu")
-        model = eval_sde_adv.SDE_Adv_Model(args, config)
-        assert type(model.runner).__module__ == "diffpure_b200.runners.diffpure_sde"
-        assert model.runner.model.kind == "ncsnpp" and hasattr(model.runner, "rev_vpsde")
-        rs._load_score_sde_state = rs_load
+        runner = getattr(runners(c["module"]), c["class"])(*[value[a] for a in c["args"]],
+                                                            **{k: value[v] for k, v in c["kwargs"].items()})
     finally:
-        for k in list(sys.modules):
-            if k == "runners" or k.startswith("runners.") or k == "eval_sde_adv":
-                sys.modules.pop(k, None)
-        for k, v in saved.items():
-            if v is not None:
-                sys.modules[k] = v
+        rs._load_score_sde_state = rs_load
+    assert type(runner).__module__ == "diffpure_b200.runners.diffpure_sde"
+    assert runner.model.kind == "ncsnpp" and hasattr(runner, "rev_vpsde")
