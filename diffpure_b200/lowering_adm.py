@@ -10,10 +10,8 @@ State-dict names are the reference's.
 """
 from types import SimpleNamespace
 
-import torch
-
-from .lowering_common import Act, act_seg, lower_attention, lower_attention_bwd, new_act, pack_conv1x1, pack_conv3x3, \
-    pack_conv_in, pack_dgrad3x3, pad_rows
+from .lowering_common import Act, AttnBlock, ResBlock, lower_attn_block, lower_data_gradient, lower_input_conv, \
+    lower_output_head, lower_resblock, lower_time_embedding, pack_conv1x1
 from .program import Program, view
 
 EPS = 1e-5
@@ -116,112 +114,46 @@ def param_shapes(cfg):
     return sh
 
 
-def lower(cfg, sd, B, h_bf16=True, tape=None):
-    """h_bf16: the first conv's output (read only by the second GroupNorm) is stored in bf16.
-    tape: a list -> every block appends the tensors its data-gradient needs and the program stops in front of the output
+def lower(cfg, sd, B, tape=None):
+    """tape: a list -> every block appends the tensors its data-gradient needs and the program stops in front of the output
     GroupNorm / conv (`lower_vjp` appends the backward ops)."""
     S = cfg.image_size
     prog = Program(B, S, S)
-    mc, emb_dim = cfg.model_channels, cfg.model_channels * 4
-    inp, mid, out, ch_final = block_plan(cfg)
+    inp, mid, out, _ = block_plan(cfg)
 
     def P(name):
         return sd[name].detach().float().cpu()
 
-    # ---- time embedding MLP + every ResBlock's FiLM projection Linear(SiLU(emb)) in one GEMM -----------
-    film_off, off = {}, 0
-    ws, bs = [], []
-    for p, kind, kw in _all_layers(cfg):
-        if kind == "res":
-            film_off[p] = off
-            off += 2 * kw["cout"]
-            ws.append(P(p + "emb_layers.1.weight"))
-            bs.append(P(p + "emb_layers.1.bias"))
-    n_all = (off + 127) // 128 * 128
-    w_all = pad_rows(torch.cat(ws, 0))
-    b_all = torch.cat(bs + [torch.zeros(n_all - off)], 0)
-    emb = prog.tensor("temb.emb", B * mc, "bf16")
-    prog.embed(emb, B, mc, cos_first=1, half_minus_1=0)                            # nn.py:111-129
-    t1 = prog.tensor("temb.h1", B * emb_dim, "bf16")
-    prog.gemm([act_seg(emb, mc)], prog.const_bf16("temb.w0", P("time_embed.0.weight")), emb_dim, mc, 1, 1, B, emb_dim,
-              bias=prog.const_f32("temb.b0", P("time_embed.0.bias")), silu=1, out_bf16=t1)
-    t2 = prog.tensor("temb.h2", B * emb_dim, "bf16")
-    prog.gemm([act_seg(t1, emb_dim)], prog.const_bf16("temb.w1", P("time_embed.2.weight")), emb_dim, emb_dim, 1, 1, B,
-              emb_dim, bias=prog.const_f32("temb.b1", P("time_embed.2.bias")), silu=1, out_bf16=t2)
-    film_all = prog.tensor("temb.film", B * n_all, "f32")
-    prog.gemm([act_seg(t2, emb_dim)], prog.const_bf16("temb.wall", w_all), n_all, emb_dim, 1, 1, B, n_all,
-              bias=prog.const_f32("temb.ball", b_all), out_f32=film_all)
+    def pair(p, a="weight", b="bias"):
+        return P(p + a), P(p + b)
+
+    # ---- time embedding MLP (nn.py:111-129) + every ResBlock's FiLM projection Linear(SiLU(emb)) in one GEMM -----------
+    res_p = [p for p, kind, _ in _all_layers(cfg) if kind == "res"]
+    film_all, offs, film_ld = lower_time_embedding(prog, B, pair("time_embed.0."), pair("time_embed.2."),
+                                                   [pair(p + "emb_layers.1.") for p in res_p], cos_first=1, half_minus_1=0)
+    film_off = dict(zip(res_p, offs))
 
     def resblock(p, kw, x0: Act, x1: Act = None):
         """ResBlock._forward, unet.py:244-264 (scale-shift norm; up/down applied after norm+act, before the conv)."""
-        cin, cout, mode = kw["cin"], kw["cout"], kw["mode"]
-        assert cin == x0.C + (x1.C if x1 else 0)
-        H, W = x0.H, x0.W
-        Ho, Wo = (H * 2, W * 2) if mode == 1 else ((H // 2, W // 2) if mode == 2 else (H, W))
-        shortcut = cin != cout
-        a0 = prog.tensor(p + "a0", B * Ho * Wo * cin, "bf16")
-        xb = prog.tensor(p + "xb", B * Ho * Wo * cin, "bf16") if shortcut else None
-        xr = prog.tensor(p + "xr", B * Ho * Wo * cin, "f32") if (mode != 0 and not shortcut) else None
-        prog.gn_apply(src0=x0.t, stats0=x0.stats, C0=x0.C, P0=x0.P, src1=x1.t if x1 else None,
-                      stats1=x1.stats if x1 else None, C1=x1.C if x1 else 0, P1=x1.P if x1 else 0,
-                      gamma=prog.const_f32(p + "n0.w", P(p + "in_layers.0.weight")),
-                      beta=prog.const_f32(p + "n0.b", P(p + "in_layers.0.bias")), B=B, H=H, W=W, groups=32, eps=EPS,
-                      silu=1, resample=mode, out_bf16=a0, raw_bf16=xb, raw_f32=xr)
-        h = new_act(prog, p + "h", B, cout, Ho, Wo)
-        if h_bf16:
-            h.t = prog.tensor(p + "h16", B * Ho * Wo * cout, "bf16")
-        prog.gemm([act_seg(a0, cin, taps=9)], prog.const_bf16(p + "w0", pack_conv3x3(P(p + "in_layers.2.weight"))),
-                  cout, 9 * cin, B, Ho, Wo, cout, bias=prog.const_f32(p + "b0", P(p + "in_layers.2.bias")),
-                  out_f32=None if h_bf16 else h.t, out_bf16=h.t if h_bf16 else None, stats=h.stats)
-        a1 = prog.tensor(p + "a1", B * Ho * Wo * cout, "bf16")
-        prog.gn_apply(src0=h.t, stats0=h.stats, C0=cout, P0=h.P,
-                      gamma=prog.const_f32(p + "n1.w", P(p + "out_layers.0.weight")),
-                      beta=prog.const_f32(p + "n1.b", P(p + "out_layers.0.bias")),
-                      film=view(film_all, film_off[p]), film_ld=n_all, B=B, H=Ho, W=Wo, groups=32, eps=EPS, silu=1,
-                      out_bf16=a1)
-        out_ = new_act(prog, p + "out", B, cout, Ho, Wo)
-        w1 = pack_conv3x3(P(p + "out_layers.3.weight"))
-        if shortcut:
-            w = torch.cat([w1, pack_conv1x1(P(p + "skip_connection.weight"))], dim=1)
-            bias = P(p + "out_layers.3.bias") + P(p + "skip_connection.bias")
-            prog.gemm([act_seg(a1, cout, taps=9), act_seg(xb, cin)], prog.const_bf16(p + "w1", w), cout,
-                      9 * cout + cin, B, Ho, Wo, cout, bias=prog.const_f32(p + "b1", bias), out_f32=out_.t,
-                      stats=out_.stats)
-        else:
-            prog.gemm([act_seg(a1, cout, taps=9)], prog.const_bf16(p + "w1", w1), cout, 9 * cout, B, Ho, Wo, cout,
-                      bias=prog.const_f32(p + "b1", P(p + "out_layers.3.bias")), resid=xr if xr is not None else x0.t,
-                      out_f32=out_.t, stats=out_.stats)
-        if tape is not None:
-            assert shortcut or x1 is None, "an identity residual over a channel concat does not occur in ADM"
-            tape.append(dict(kind="res", p=p, kw=kw, x0=x0, x1=x1, h=h, out=out_, shortcut=shortcut, Ho=Ho, Wo=Wo,
-                             film=view(film_all, film_off[p]), film_ld=n_all))
-        return out_
+        cin, cout = kw["cin"], kw["cout"]
+        blk = ResBlock(p[:-1], cin, cout, gn0=pair(p + "in_layers.0."), conv0=pair(p + "in_layers.2."),
+                       gn1=pair(p + "out_layers.0."), conv1=pair(p + "out_layers.3."),
+                       skip=pair(p + "skip_connection.") if cin != cout else None, temb=view(film_all, film_off[p]),
+                       temb_ld=film_ld, film=True, groups0=32, groups1=32, eps=EPS, resample=kw["mode"])
+        return lower_resblock(prog, blk, B, x0, x1, tape=tape)
 
-    def attnblock(p, kw, x: Act):
+    def attnblock(p, x: Act):
         """AttentionBlock._forward + QKVAttentionLegacy, unet.py:307-313,345-362."""
-        C, H, W = x.C, x.H, x.W
-        T = H * W
+        C = x.C
         d = cfg.num_head_channels
         heads = C // d
-        hn = prog.tensor(p + "hn", B * T * C, "bf16")
-        prog.gn_apply(src0=x.t, stats0=x.stats, C0=C, P0=x.P, gamma=prog.const_f32(p + "n.w", P(p + "norm.weight")),
-                      beta=prog.const_f32(p + "n.b", P(p + "norm.bias")), B=B, H=H, W=W, groups=32, eps=EPS, silu=0,
-                      out_bf16=hn)
         # legacy packing: output channel h*3d + {0,1,2}*d + c  ->  head-major q | k | v blocks
         wqkv = P(p + "qkv.weight").reshape(heads, 3, d, C)
         bqkv = P(p + "qkv.bias").reshape(heads, 3, d)
-        wq, wk, wv = (wqkv[:, j].reshape(C, C).contiguous() for j in range(3))
-        bq, bk, bv = (bqkv[:, j].reshape(C).contiguous() for j in range(3))
-        rec = dict(kind="attn", p=p, x=x, T=T, C=C, heads=heads, scale=float(d) ** (-0.5), wqkv=(wq, wk, wv)) \
-            if tape is not None else None
-        o = lower_attention(prog, p + "att", hn, wq, wk, wv, bq, bk, bv, B, T, C, heads, float(d) ** (-0.5), rec=rec)
-        out_ = new_act(prog, p + "out", B, C, H, W)
-        prog.gemm([act_seg(o, C)], prog.const_bf16(p + "wo", pack_conv1x1(P(p + "proj_out.weight"))), C, C, B, H, W, C,
-                  bias=prog.const_f32(p + "bo", P(p + "proj_out.bias")), resid=x.t, out_f32=out_.t, stats=out_.stats)
-        if tape is not None:
-            rec["out"] = out_
-            tape.append(rec)
-        return out_
+        q, k, v = ((wqkv[:, j].reshape(C, C).contiguous(), bqkv[:, j].reshape(C).contiguous()) for j in range(3))
+        blk = AttnBlock(p[:-1], pair(p + "norm."), q, k, v, (pack_conv1x1(P(p + "proj_out.weight")), P(p + "proj_out.bias")),
+                        heads=heads, scale=float(d) ** (-0.5), groups=32, eps=EPS)
+        return lower_attn_block(prog, blk, B, x, tape=tape)
 
     def run(prefix, layers, x0, x1=None):
         h = x0
@@ -231,15 +163,12 @@ def lower(cfg, sd, B, h_bf16=True, tape=None):
                 h = resblock(p, kw, h, x1)
                 x1 = None
             else:
-                h = attnblock(p, kw, h)
+                h = attnblock(p, h)
         return h
 
     # ---- UNetModel.forward, unet.py:642-671 ---------------------------------------------------------------
-    ch0 = inp[0][0][1]["cout"]
-    h = new_act(prog, "conv_in.out", B, ch0, S, S)
-    prog.conv_in_gemm("conv_in", P("input_blocks.0.0.weight"), P("input_blocks.0.0.bias"), h.t, h.stats, B, S, S, ch0)
+    h = lower_input_conv(prog, pair("input_blocks.0.0."), B, tape)
     hs = [h]
-    hs0 = h
     for i, layers in enumerate(inp[1:], start=1):
         h = run(f"input_blocks.{i}.", layers, h)
         hs.append(h)
@@ -247,16 +176,7 @@ def lower(cfg, sd, B, h_bf16=True, tape=None):
     for i, layers in enumerate(out):
         h = run(f"output_blocks.{i}.", layers, h, hs.pop())
     assert not hs
-    if tape is not None:
-        tape.append(dict(kind="gn_out", x=h))
-        tape.insert(0, dict(kind="conv_in", out=hs0))
-        prog.meta.update(model="adm", out_channels=cfg.out_channels, cond="timestep")
-        return prog
-    a = prog.tensor("out.a", B * S * S * h.C, "bf16")
-    prog.gn_apply(src0=h.t, stats0=h.stats, C0=h.C, P0=h.P, gamma=prog.const_f32("out.n.w", P("out.0.weight")),
-                  beta=prog.const_f32("out.n.b", P("out.0.bias")), B=B, H=S, W=S, groups=32, eps=EPS, silu=1,
-                  out_bf16=a)
-    prog.conv_out_gemm("out", a, P("out.2.weight"), P("out.2.bias"), B, S, S, h.C, cfg.out_channels)
+    lower_output_head(prog, h, pair("out.0."), 32, EPS, pair("out.2."), B, tape)
     prog.meta.update(model="adm", out_channels=cfg.out_channels, cond="timestep")
     return prog
 
@@ -267,106 +187,9 @@ def lower_vjp(cfg, sd, B, g_channels=3):
     runners/diffpure_sde.py:96-122 reads; 6 = eps and the learned-variance half).
 
     The reference differentiates this network through torchsde's adjoint for the ImageNet white-box attacks
-    (run_scripts/imagenet/run_in_rand_inf.sh -> eval_sde_adv.py:126-128 -> runners/diffpure_sde.py:233-239). Every conv is
-    the same tcgen05 implicit GEMM with flipped / transposed weights; GroupNorm(+SiLU, +scale-shift, +up / down resample,
-    +concat) is the two-pass `gn_bwd` op (the per-sample scale-shift rows fold into gamma / beta); attention is
-    `lower_attention_bwd` (multi-head, T = 1024 / 256 / 64). Gradient stream fp32, GEMM operands bf16. Held against
-    torch.autograd on the reference-pinned oracle forward (tests/test_vjp_lowering_cpu.py)."""
+    (run_scripts/imagenet/run_in_rand_inf.sh -> eval_sde_adv.py:126-128 -> runners/diffpure_sde.py:233-239). The
+    per-sample scale-shift rows fold into gn_bwd's gamma / beta; attention is multi-head at T = 1024 / 256 / 64. Held
+    against torch.autograd on the reference-pinned oracle forward (tests/test_vjp_lowering_cpu.py)."""
     tape = []
     prog = lower(cfg, sd, B, tape=tape)
-    S = cfg.image_size
-
-    def P(name):
-        return sd[name].detach().float().cpu()
-
-    grad = {}        # tensor index -> (fp32 gradient, bf16 copy) of a residual-stream tensor
-    skip_grad = {}   # tensor index -> fp32 gradient that reached the tensor through its skip connection
-
-    def gpair(name, n):
-        return prog.tensor(name + ".g32", n, "f32"), prog.tensor(name + ".g16", n, "bf16")
-
-    # ---- output conv (the first g_channels output channels) + output GroupNorm ----------------------------------------
-    hl = tape[-1]["x"]
-    C = hl.C
-    gin = prog.tensor("bwd.gin", B * S * S * 64, "bf16")
-    prog.grad_in(gin, B, S, S, g_channels, 64)
-    wout = torch.zeros(64, C, 3, 3)
-    wout[:g_channels] = P("out.2.weight")[:g_channels]
-    ga = prog.tensor("bwd.out.ga", B * S * S * C, "f32")
-    prog.gemm([act_seg(gin, 64, taps=9)], prog.const_bf16("bwd.out.w", pack_dgrad3x3(wout)), C, 9 * 64, B, S, S, C,
-              out_f32=ga)
-    g32, g16 = gpair("bwd.out", B * S * S * C)
-    prog.gn_bwd(src0=hl.t, stats0=hl.stats, C0=C, P0=hl.P, gamma=prog.const_f32("bwd.out.n.w", P("out.0.weight")),
-                beta=prog.const_f32("bwd.out.n.b", P("out.0.bias")), B=B, H=S, W=S, groups=32, eps=EPS, silu=1, g=ga,
-                d0_f32=g32, d0_bf16=g16)
-    grad[hl.t.index] = (g32, g16)
-
-    def res_bwd(r):
-        """ResBlock._forward backwards (unet.py:244-264): out = skip(x') + conv1(silu(FiLM(GN1(conv0(silu(GN0(x))'))))),
-        ' = the up / down resample."""
-        p, kw, x0, x1, h, Ho, Wo = r["p"], r["kw"], r["x0"], r["x1"], r["h"], r["Ho"], r["Wo"]
-        cin, cout, mode = kw["cin"], kw["cout"], kw["mode"]
-        H, W = x0.H, x0.W
-        name = "bwd." + p
-        g32, g16 = grad.pop(r["out"].t.index)
-        ga1 = prog.tensor(name + "ga1", B * Ho * Wo * cout, "f32")
-        prog.gemm([act_seg(g16, cout, taps=9)], prog.const_bf16(name + "w1", pack_dgrad3x3(P(p + "out_layers.3.weight"))),
-                  cout, 9 * cout, B, Ho, Wo, cout, out_f32=ga1)
-        gc0 = prog.tensor(name + "gc0", B * Ho * Wo * cout, "bf16")
-        prog.gn_bwd(src0=h.t, stats0=h.stats, C0=cout, P0=h.P, gamma=prog.const_f32(name + "n1.w", P(p + "out_layers.0.weight")),
-                    beta=prog.const_f32(name + "n1.b", P(p + "out_layers.0.bias")), film=r["film"], film_ld=r["film_ld"],
-                    B=B, H=Ho, W=Wo, groups=32, eps=EPS, silu=1, g=ga1, d0_bf16=gc0)
-        ga0 = prog.tensor(name + "ga0", B * Ho * Wo * cin, "f32")
-        prog.gemm([act_seg(gc0, cout, taps=9)], prog.const_bf16(name + "w0", pack_dgrad3x3(P(p + "in_layers.2.weight"))),
-                  cin, 9 * cout, B, Ho, Wo, cin, out_f32=ga0)
-        if r["shortcut"]:
-            gxs = prog.tensor(name + "gxs", B * Ho * Wo * cin, "f32")
-            prog.gemm([act_seg(g16, cout)],
-                      prog.const_bf16(name + "ws", pack_conv1x1(P(p + "skip_connection.weight")).t().contiguous()), cin, cout,
-                      B, Ho, Wo, cin, out_f32=gxs)
-            add0 = gxs
-        else:
-            add0 = g32
-        d32, d16 = gpair(name + "dx", B * H * W * x0.C)
-        d1 = prog.tensor(name + "dskip", B * H * W * x1.C, "f32") if x1 else None
-        prog.gn_bwd(src0=x0.t, stats0=x0.stats, C0=x0.C, P0=x0.P, src1=x1.t if x1 else None,
-                    stats1=x1.stats if x1 else None, C1=x1.C if x1 else 0, P1=x1.P if x1 else 0,
-                    gamma=prog.const_f32(name + "n0.w", P(p + "in_layers.0.weight")),
-                    beta=prog.const_f32(name + "n0.b", P(p + "in_layers.0.bias")), B=B, H=H, W=W, groups=32, eps=EPS,
-                    silu=1, resample=mode, g=ga0, add0=add0, add0_scale=1.0, add1=skip_grad.pop(x0.t.index, None),
-                    d0_f32=d32, d0_bf16=d16, d1_f32=d1)
-        grad[x0.t.index] = (d32, d16)
-        if x1:
-            skip_grad[x1.t.index] = d1
-
-    def attn_bwd(r):
-        """AttentionBlock._forward backwards (unet.py:307-313): out = x + proj_out(attention(qkv(norm(x))))."""
-        p, x, T, C = r["p"], r["x"], r["T"], r["C"]
-        H, W = x.H, x.W
-        name = "bwd." + p
-        g32, g16 = grad.pop(r["out"].t.index)
-        go = prog.tensor(name + "go", B * T * C, "bf16")
-        prog.gemm([act_seg(g16, C)], prog.const_bf16(name + "wo", pack_conv1x1(P(p + "proj_out.weight")).t().contiguous()),
-                  C, C, 1, 1, B * T, C, out_bf16=go)
-        dqkv = lower_attention_bwd(prog, name + "att", r, go, B, T, C, r["heads"], r["scale"])
-        ghn = prog.tensor(name + "ghn", B * T * C, "f32")
-        wqkv = torch.cat(r["wqkv"], 0).t().contiguous()                       # [C_in, 3 C_out]
-        prog.gemm([act_seg(dqkv, 3 * C)], prog.const_bf16(name + "wqkv", wqkv), C, 3 * C, 1, 1, B * T, C, out_f32=ghn)
-        d32, d16 = gpair(name + "dx", B * T * C)
-        prog.gn_bwd(src0=x.t, stats0=x.stats, C0=C, P0=x.P, gamma=prog.const_f32(name + "n.w", P(p + "norm.weight")),
-                    beta=prog.const_f32(name + "n.b", P(p + "norm.bias")), B=B, H=H, W=W, groups=32, eps=EPS, silu=0,
-                    g=ghn, add0=g32, add0_scale=1.0, add1=skip_grad.pop(x.t.index, None), d0_f32=d32, d0_bf16=d16)
-        grad[x.t.index] = (d32, d16)
-
-    for r in reversed(tape[1:-1]):
-        (res_bwd if r["kind"] == "res" else attn_bwd)(r)
-    h0 = tape[0]["out"]
-    _, g16 = grad.pop(h0.t.index)
-    assert not grad and not skip_grad, (list(grad), list(skip_grad))
-    ch0 = h0.C
-    gx8 = prog.tensor("bwd.gx8", B * S * S * 8, "f32")
-    prog.gemm([act_seg(g16, ch0, taps=9)], prog.const_bf16("bwd.conv_in.w", pack_dgrad3x3(P("input_blocks.0.0.weight"))),
-              3, 9 * ch0, B, S, S, 8, out_f32=gx8, ldc=8)
-    prog.update(gx8, 8, B, S, S, 3)
-    prog.meta.update(vjp=True)
-    return prog
+    return lower_data_gradient(prog, tape, B, g_channels)

@@ -7,10 +7,8 @@ State-dict names are the reference's.
 """
 from types import SimpleNamespace
 
-import torch
-
-from .lowering_common import Act, act_seg, lower_attention, new_act, pack_conv1x1, pack_conv3x3, pack_conv_in, \
-    pad_rows
+from .lowering_common import Act, AttnBlock, ResBlock, act_seg, lower_attn_block, lower_input_conv, lower_output_head, \
+    lower_resblock, lower_time_embedding, new_act, pack_conv1x1, pack_conv3x3
 from .program import Program, view
 
 EPS = 1e-6
@@ -97,90 +95,38 @@ def param_shapes(cfg):
     return sh
 
 
-def lower(cfg, sd, B, h_bf16=True):
-    """h_bf16: conv1's output (read only by norm2) is stored in bf16."""
+def lower(cfg, sd, B):
     S = cfg.image_size
     prog = Program(B, S, S)
-    ch, temb_dim = cfg.ch, cfg.ch * 4
     nres = len(cfg.ch_mult)
 
     def P(name):
         return sd[name].detach().float().cpu()
 
-    # ---- timestep embedding MLP + all temb_proj(swish(temb)) in one GEMM ------------------------------
+    def pair(p, a="weight", b="bias"):
+        return P(p + a), P(p + b)
+
+    # ---- timestep embedding MLP (L14-32) + all temb_proj(swish(temb)) in one GEMM --------------------------------
     blocks = block_list(cfg)
-    dense_off, off = {}, 0
-    for p, cin, cout in blocks:
-        dense_off[p] = off
-        off += cout
-    n_all = (off + 127) // 128 * 128
-    w_all = pad_rows(torch.cat([P(p + "temb_proj.weight") for p, _, _ in blocks], 0))
-    b_all = torch.cat([P(p + "temb_proj.bias") for p, _, _ in blocks] + [torch.zeros(n_all - off)], 0)
-    emb = prog.tensor("temb.emb", B * ch, "bf16")
-    prog.embed(emb, B, ch, cos_first=0, half_minus_1=1)
-    t1 = prog.tensor("temb.h1", B * temb_dim, "bf16")
-    prog.gemm([act_seg(emb, ch)], prog.const_bf16("temb.w0", P("temb.dense.0.weight")), temb_dim, ch, 1, 1, B, temb_dim,
-              bias=prog.const_f32("temb.b0", P("temb.dense.0.bias")), silu=1, out_bf16=t1)
-    t2 = prog.tensor("temb.h2", B * temb_dim, "bf16")
-    prog.gemm([act_seg(t1, temb_dim)], prog.const_bf16("temb.w1", P("temb.dense.1.weight")), temb_dim, temb_dim, 1, 1,
-              B, temb_dim, bias=prog.const_f32("temb.b1", P("temb.dense.1.bias")), silu=1, out_bf16=t2)
-    temb_all = prog.tensor("temb.all", B * n_all, "f32")
-    prog.gemm([act_seg(t2, temb_dim)], prog.const_bf16("temb.wall", w_all), n_all, temb_dim, 1, 1, B, n_all,
-              bias=prog.const_f32("temb.ball", b_all), out_f32=temb_all)
+    temb_all, offs, temb_ld = lower_time_embedding(prog, B, pair("temb.dense.0."), pair("temb.dense.1."),
+                                                   [pair(p + "temb_proj.") for p, _, _ in blocks], cos_first=0,
+                                                   half_minus_1=1)
+    temb_off = {p: off for (p, _, _), off in zip(blocks, offs)}
 
     def resblock(p, x0: Act, x1: Act = None):
         """ResnetBlock.forward, unet_ddpm.py:123-142."""
         cin = x0.C + (x1.C if x1 else 0)
         cout = P(p + "conv1.weight").shape[0]
-        H, W = x0.H, x0.W
-        shortcut = cin != cout
-        a0 = prog.tensor(p + "a0", B * H * W * cin, "bf16")
-        xb = prog.tensor(p + "xb", B * H * W * cin, "bf16") if shortcut else None
-        prog.gn_apply(src0=x0.t, stats0=x0.stats, C0=x0.C, P0=x0.P, src1=x1.t if x1 else None,
-                      stats1=x1.stats if x1 else None, C1=x1.C if x1 else 0, P1=x1.P if x1 else 0,
-                      gamma=prog.const_f32(p + "n1.w", P(p + "norm1.weight")),
-                      beta=prog.const_f32(p + "n1.b", P(p + "norm1.bias")), B=B, H=H, W=W, groups=32, eps=EPS, silu=1,
-                      out_bf16=a0, raw_bf16=xb)
-        h = new_act(prog, p + "h", B, cout, H, W)
-        if h_bf16:
-            h.t = prog.tensor(p + "h16", B * H * W * cout, "bf16")
-        prog.gemm([act_seg(a0, cin, taps=9)], prog.const_bf16(p + "w1", pack_conv3x3(P(p + "conv1.weight"))), cout,
-                  9 * cin, B, H, W, cout, bias=prog.const_f32(p + "b1", P(p + "conv1.bias")),
-                  rowvec=view(temb_all, dense_off[p]), rowvec_ld=n_all, rowvec_rows_per_sample=H * W,
-                  out_f32=None if h_bf16 else h.t, out_bf16=h.t if h_bf16 else None, stats=h.stats)
-        a1 = prog.tensor(p + "a1", B * H * W * cout, "bf16")
-        prog.gn_apply(src0=h.t, stats0=h.stats, C0=cout, P0=h.P,
-                      gamma=prog.const_f32(p + "n2.w", P(p + "norm2.weight")),
-                      beta=prog.const_f32(p + "n2.b", P(p + "norm2.bias")), B=B, H=H, W=W, groups=32, eps=EPS, silu=1,
-                      out_bf16=a1)
-        out = new_act(prog, p + "out", B, cout, H, W)
-        w2 = pack_conv3x3(P(p + "conv2.weight"))
-        if shortcut:
-            w = torch.cat([w2, pack_conv1x1(P(p + "nin_shortcut.weight"))], dim=1)
-            bias = P(p + "conv2.bias") + P(p + "nin_shortcut.bias")
-            prog.gemm([act_seg(a1, cout, taps=9), act_seg(xb, cin)], prog.const_bf16(p + "w2", w), cout,
-                      9 * cout + cin, B, H, W, cout, bias=prog.const_f32(p + "b2", bias), out_f32=out.t,
-                      stats=out.stats)
-        else:
-            prog.gemm([act_seg(a1, cout, taps=9)], prog.const_bf16(p + "w2", w2), cout, 9 * cout, B, H, W, cout,
-                      bias=prog.const_f32(p + "b2", P(p + "conv2.bias")), resid=x0.t, out_f32=out.t, stats=out.stats)
-        return out
+        blk = ResBlock(p[:-1], cin, cout, gn0=pair(p + "norm1."), conv0=pair(p + "conv1."), gn1=pair(p + "norm2."),
+                       conv1=pair(p + "conv2."), skip=pair(p + "nin_shortcut.") if cin != cout else None,
+                       temb=view(temb_all, temb_off[p]), temb_ld=temb_ld, film=False, groups0=32, groups1=32, eps=EPS)
+        return lower_resblock(prog, blk, B, x0, x1)
 
     def attnblock(p, x: Act):
         """AttnBlock.forward, unet_ddpm.py:172-197."""
-        C, H, W = x.C, x.H, x.W
-        T = H * W
-        hn = prog.tensor(p + "hn", B * T * C, "bf16")
-        prog.gn_apply(src0=x.t, stats0=x.stats, C0=C, P0=x.P, gamma=prog.const_f32(p + "n.w", P(p + "norm.weight")),
-                      beta=prog.const_f32(p + "n.b", P(p + "norm.bias")), B=B, H=H, W=W, groups=32, eps=EPS, silu=0,
-                      out_bf16=hn)
-        o = lower_attention(prog, p + "att", hn, pack_conv1x1(P(p + "q.weight")), pack_conv1x1(P(p + "k.weight")),
-                            pack_conv1x1(P(p + "v.weight")), P(p + "q.bias"), P(p + "k.bias"), P(p + "v.bias"), B, T, C,
-                            1, int(C) ** (-0.5))
-        out = new_act(prog, p + "out", B, C, H, W)
-        prog.gemm([act_seg(o, C)], prog.const_bf16(p + "wo", pack_conv1x1(P(p + "proj_out.weight"))), C, C, B, H, W, C,
-                  bias=prog.const_f32(p + "bo", P(p + "proj_out.bias")), resid=x.t, out_f32=out.t, stats=out.stats)
-        return out
+        q, k, v, o = ((pack_conv1x1(P(p + n + ".weight")), P(p + n + ".bias")) for n in ("q", "k", "v", "proj_out"))
+        blk = AttnBlock(p[:-1], pair(p + "norm."), q, k, v, o, heads=1, scale=int(x.C) ** (-0.5), groups=32, eps=EPS)
+        return lower_attn_block(prog, blk, B, x)
 
     def resample_conv(p, x: Act, mode):
         """Downsample (pad right/bottom + 3x3 stride 2) / Upsample (nearest x2 + 3x3) on the raw stream."""
@@ -201,8 +147,7 @@ def lower(cfg, sd, B, h_bf16=True):
         return out
 
     # ---- Model.forward, unet_ddpm.py:305-345 -------------------------------------------------------------
-    h0 = new_act(prog, "conv_in.out", B, ch, S, S)
-    prog.conv_in_gemm("conv_in", P("conv_in.weight"), P("conv_in.bias"), h0.t, h0.stats, B, S, S, ch)
+    h0 = lower_input_conv(prog, pair("conv_in."), B)
     hs = [h0]
     res = S
     for lvl in range(nres):
@@ -227,10 +172,6 @@ def lower(cfg, sd, B, h_bf16=True):
             h = resample_conv(f"up.{lvl}.upsample.", h, "up")
             res *= 2
     assert not hs
-    a = prog.tensor("out.a", B * S * S * h.C, "bf16")
-    prog.gn_apply(src0=h.t, stats0=h.stats, C0=h.C, P0=h.P, gamma=prog.const_f32("out.n.w", P("norm_out.weight")),
-                  beta=prog.const_f32("out.n.b", P("norm_out.bias")), B=B, H=S, W=S, groups=32, eps=EPS, silu=1,
-                  out_bf16=a)
-    prog.conv_out_gemm("out", a, P("conv_out.weight"), P("conv_out.bias"), B, S, S, h.C, cfg.out_ch)
+    lower_output_head(prog, h, pair("norm_out."), 32, EPS, pair("conv_out."), B)
     prog.meta.update(model="ddpm", out_channels=cfg.out_ch, cond="timestep")
     return prog

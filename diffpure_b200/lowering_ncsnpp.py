@@ -16,11 +16,11 @@ All per-block Dense_0(SiLU(temb)) projections are one GEMM per step.
 import os
 from types import SimpleNamespace
 
-import torch
-
-from .lowering_common import INV_SQRT2, Act, act_seg, new_act, pack_conv1x1, pack_conv3x3, pack_conv_in, pack_dgrad3x3, \
-    pad_rows, transposed as _transposed
+from .lowering_common import INV_SQRT2, Act, AttnBlock, ResBlock, const_pair, lower_attn_block, lower_data_gradient, \
+    lower_input_conv, lower_output_head, lower_resblock, lower_time_embedding, pack_dgrad3x3  # noqa: F401 (re-export)
 from .program import Program, view
+
+EPS = 1e-6
 
 
 def cifar10_cfg():
@@ -110,256 +110,107 @@ def param_shapes(cfg):
     return shapes
 
 
-def lower(cfg, sd, B, h_bf16=True, tape=None, fuse_gn=True, fuse_attn=True):
+def lower(cfg, sd, B, tape=None, fuse_attn=True):
     """Build the engine program for batch size B. `sd`: name -> fp32 torch tensor (CPU).
-    h_bf16: store the Conv_0 output (only ever read by GroupNorm_1) in bf16 -- halves its HBM round trip; the
-    GroupNorm statistics are still accumulated from the fp32 accumulator values.
-    fuse_gn: GroupNorm_1 + act of every res-block in the epilogue of its Conv_0 GEMM (the conv result stays in TMEM).
+    Every res-block's GroupNorm_1 + act runs in the epilogue of its Conv_0 GEMM, and a block's output GroupNorm + act is
+    written by its producer's epilogue wherever `consumer_gn` allows it.
     fuse_attn: an attention block of T = 256 tokens x C = 256 channels (the 16x16 level of the CIFAR-10 model) as ONE
     kernel (`attn_block`, dp_attn.cu) instead of five GEMM launches; DP_FUSE_ATTN=0 in the environment turns it off (A/B).
-    tape: a list -> every block appends the tensors its data-gradient needs and the program stops in front of the
-    output GroupNorm / conv (`lower_vjp` appends the backward ops)."""
+    tape: a list -> every block appends the tensors its data-gradient needs, no fusion, and the program stops in front
+    of the output GroupNorm / conv (`lower_vjp` appends the backward ops)."""
     S = cfg.image_size
     prog = Program(B, S, S)
     plan = module_plan(cfg)
-    nf = cfg.nf
-    temb_dim = 4 * nf
-    fuse_attn = fuse_attn and os.environ.get("DP_FUSE_ATTN", "1") != "0"
+    fuse = tape is None
+    fuse_attn = fuse and fuse_attn and os.environ.get("DP_FUSE_ATTN", "1") != "0"
 
     def P(i, name):
         return sd[f"all_modules.{i}.{name}"].detach().float().cpu()
 
-    # ---- time embedding MLP + all per-block Dense_0 projections in one GEMM -------------------------
-    dense_off = {}
-    dense_w, dense_b = [], []
-    off = 0
-    for i, (kind, kw) in enumerate(plan):
-        if kind == "res":
-            dense_off[i] = off
-            dense_w.append(P(i, "Dense_0.weight"))
-            dense_b.append(P(i, "Dense_0.bias"))
-            off += kw["cout"]
-    n_all = (off + 127) // 128 * 128
-    w_all = pad_rows(torch.cat(dense_w, 0))
-    b_all = torch.cat(dense_b + [torch.zeros(n_all - off)], 0)
+    def pair(i, a, b):
+        return P(i, a), P(i, b)
 
-    emb = prog.tensor("temb.emb", B * nf, "bf16")
-    prog.embed(emb, B, nf, cos_first=0, half_minus_1=1)                      # layers.py:515-529
-    t1 = prog.tensor("temb.h1", B * temb_dim, "bf16")
-    prog.gemm([act_seg(emb, nf)], prog.const_bf16("temb.w0", P(0, "weight")), temb_dim, nf, 1, 1, B, temb_dim,
-              bias=prog.const_f32("temb.b0", P(0, "bias")), silu=1, out_bf16=t1)   # ncsnpp.py:252-254
-    t2 = prog.tensor("temb.h2", B * temb_dim, "bf16")
-    prog.gemm([act_seg(t1, temb_dim)], prog.const_bf16("temb.w1", P(1, "weight")), temb_dim, temb_dim, 1, 1, B,
-              temb_dim, bias=prog.const_f32("temb.b1", P(1, "bias")), silu=1, out_bf16=t2)  # SiLU: every consumer
-    temb_all = prog.tensor("temb.all", B * n_all, "f32")                      # applies act(temb), layerspp.py:263
-    prog.gemm([act_seg(t2, temb_dim)], prog.const_bf16("temb.wall", w_all), n_all, temb_dim, 1, 1, B, n_all,
-              bias=prog.const_f32("temb.ball", b_all), out_f32=temb_all)
+    # ---- time embedding MLP + all per-block Dense_0 projections in one GEMM (layers.py:515-529, ncsnpp.py:252-254;
+    # every consumer applies act(temb), layerspp.py:263) -------------------------------------------------------------
+    res_idx = [i for i, (kind, _) in enumerate(plan) if kind == "res"]
+    temb_all, offs, temb_ld = lower_time_embedding(
+        prog, B, pair(0, "weight", "bias"), pair(1, "weight", "bias"),
+        [pair(i, "Dense_0.weight", "Dense_0.bias") for i in res_idx], cos_first=0, half_minus_1=1)
+    temb_off = dict(zip(res_idx, offs))
 
-    # ---- the consumer of a block's output, seen from its producer ----------------------------------------
     def consumer_gn(j, C):
         """If the op after plan entry j-1 normalises the WHOLE incoming tensor (C channels) on its own -- a plain res-block
         (no up / down resample in front of Conv_0, no channel concat), an attention block or the output GroupNorm -- return
-        what the producer's epilogue needs to emit that operand itself: dict(gamma, beta, groups, silu, raw16)."""
-        if not fuse_gn or tape is not None or j >= len(plan):
+        what the producer's epilogue needs to emit that operand itself (`gn_epilogue_args`)."""
+        if not fuse or j >= len(plan):
             return None
         kind, kw = plan[j]
         if kind == "res" and kw["mode"] == 0 and kw["role"] in ("down", "mid") and kw["cin"] == C:
-            return dict(gamma=prog.const_f32(f"m{j}.gn0.w", P(j, "GroupNorm_0.weight")),
-                        beta=prog.const_f32(f"m{j}.gn0.b", P(j, "GroupNorm_0.bias")), groups=_groups(C), silu=1,
-                        raw16=kw["cin"] != kw["cout"])
+            gamma, beta = const_pair(prog, f"m{j}.gn0", pair(j, "GroupNorm_0.weight", "GroupNorm_0.bias"))
+            return dict(gamma=gamma, beta=beta, groups=_groups(C), eps=EPS, silu=1, raw16=kw["cin"] != kw["cout"])
         if kind == "attn" and kw["c"] == C:
-            return dict(gamma=prog.const_f32(f"m{j}.gn.w", P(j, "GroupNorm_0.weight")),
-                        beta=prog.const_f32(f"m{j}.gn.b", P(j, "GroupNorm_0.bias")), groups=_groups(C), silu=0, raw16=False)
+            gamma, beta = const_pair(prog, f"m{j}.gn", pair(j, "GroupNorm_0.weight", "GroupNorm_0.bias"))
+            return dict(gamma=gamma, beta=beta, groups=_groups(C), eps=EPS, silu=0, raw16=False)
         if kind == "gn_out" and kw["c"] == C:
-            return dict(gamma=prog.const_f32("out.gn.w", P(j, "weight")), beta=prog.const_f32("out.gn.b", P(j, "bias")),
-                        groups=_groups(C), silu=1, raw16=False)
+            gamma, beta = const_pair(prog, "out.gn", pair(j, "weight", "bias"))
+            return dict(gamma=gamma, beta=beta, groups=_groups(C), eps=EPS, silu=1, raw16=False)
         return None
 
-    def gn_epilogue_args(out: Act, spec, name):
-        """gemm() keyword arguments that make the producer of `out` also write its consumer's normalised operand."""
-        if spec is None:
-            return {}
-        out.pre = prog.tensor(name + ".next_a0", B * out.H * out.W * out.C, "bf16")
-        kw = dict(gn_out=out.pre, gn_gamma=spec["gamma"], gn_beta=spec["beta"], gn_groups=spec["groups"], gn_eps=1e-6,
-                  gn_silu=spec["silu"])
-        if spec["raw16"]:
-            out.raw16 = prog.tensor(name + ".next_xb", B * out.H * out.W * out.C, "bf16")
-            kw["out_bf16"] = out.raw16
-        return kw
-
-    # ---- blocks ---------------------------------------------------------------------------------------
-    def resblock(i, kw, x0: Act, x1: Act = None):
+    def resblock(i, x0: Act, x1: Act = None):
         """ResnetBlockBigGANpp.forward, layerspp.py:242-274."""
+        kw = plan[i][1]
         cin, cout, mode = kw["cin"], kw["cout"], kw["mode"]
-        assert cin == x0.C + (x1.C if x1 else 0)
-        H, W = x0.H, x0.W
-        Ho, Wo = (H * 2, W * 2) if mode == 1 else ((H // 2, W // 2) if mode == 2 else (H, W))
-        shortcut = (cin != cout) or mode != 0
-        name = f"m{i}"
-        if x0.pre is not None and x1 is None and mode == 0:
-            # GroupNorm_0 + act of this block already came out of the producer's epilogue (and the raw bf16 copy with it)
-            a0, xb = x0.pre, x0.raw16
-            assert (xb is not None) == shortcut
-        else:
-            a0 = prog.tensor(name + ".a0", B * Ho * Wo * cin, "bf16")
-            xb = prog.tensor(name + ".xb", B * Ho * Wo * cin, "bf16") if shortcut else None
-            prog.gn_apply(src0=x0.t, stats0=x0.stats, C0=x0.C, P0=x0.P,
-                          src1=x1.t if x1 else None, stats1=x1.stats if x1 else None, C1=x1.C if x1 else 0,
-                          P1=x1.P if x1 else 0,
-                          gamma=prog.const_f32(name + ".gn0.w", P(i, "GroupNorm_0.weight")),
-                          beta=prog.const_f32(name + ".gn0.b", P(i, "GroupNorm_0.bias")),
-                          B=B, H=H, W=W, groups=_groups(cin), eps=1e-6, silu=1, resample=mode, out_bf16=a0, raw_bf16=xb)
-        a1 = prog.tensor(name + ".a1", B * Ho * Wo * cout, "bf16")
-        w0 = prog.const_bf16(name + ".w0", pack_conv3x3(P(i, "Conv_0.weight")))
-        b0 = prog.const_f32(name + ".b0", P(i, "Conv_0.bias"))
-        gn1w = prog.const_f32(name + ".gn1.w", P(i, "GroupNorm_1.weight"))
-        gn1b = prog.const_f32(name + ".gn1.b", P(i, "GroupNorm_1.bias"))
-        h = None
-        if fuse_gn and tape is None:
-            # Conv_0 + Dense_0(act(temb)) + GroupNorm_1 + act in ONE kernel: the conv's result is only ever read by
-            # GroupNorm_1 (layerspp.py:259-266), so it never leaves TMEM -- the epilogue writes the normalised operand
-            prog.gemm([act_seg(a0, cin, taps=9)], w0, cout, 9 * cin, B, Ho, Wo, cout, bias=b0,
-                      rowvec=view(temb_all, dense_off[i]), rowvec_ld=n_all, rowvec_rows_per_sample=Ho * Wo,
-                      gn_out=a1, gn_gamma=gn1w, gn_beta=gn1b, gn_groups=_groups(cout), gn_eps=1e-6, gn_silu=1)
-        else:
-            h = new_act(prog, name + ".h", B, cout, Ho, Wo)
-            if h_bf16:
-                h.t = prog.tensor(name + ".h16", B * Ho * Wo * cout, "bf16")
-            prog.gemm([act_seg(a0, cin, taps=9)], w0, cout, 9 * cin, B, Ho, Wo, cout, bias=b0,
-                      rowvec=view(temb_all, dense_off[i]), rowvec_ld=n_all, rowvec_rows_per_sample=Ho * Wo,
-                      out_f32=None if h_bf16 else h.t, out_bf16=h.t if h_bf16 else None, stats=h.stats)
-            prog.gn_apply(src0=h.t, stats0=h.stats, C0=cout, P0=h.P, gamma=gn1w, beta=gn1b,
-                          B=B, H=Ho, W=Wo, groups=_groups(cout), eps=1e-6, silu=1, out_bf16=a1)
-        out = new_act(prog, name + ".out", B, cout, Ho, Wo)
-        nxt = gn_epilogue_args(out, consumer_gn(i + 1, cout), name)   # the next block's GroupNorm_0 in this epilogue
-        w1 = pack_conv3x3(P(i, "Conv_1.weight"))
-        if shortcut:
-            w = torch.cat([w1, pack_conv1x1(P(i, "Conv_2.weight"))], dim=1)
-            bias = P(i, "Conv_1.bias") + P(i, "Conv_2.bias")
-            prog.gemm([act_seg(a1, cout, taps=9), act_seg(xb, cin)], prog.const_bf16(name + ".w1", w), cout,
-                      9 * cout + cin, B, Ho, Wo, cout, bias=prog.const_f32(name + ".b1", bias), alpha=INV_SQRT2,
-                      out_f32=out.t, stats=out.stats, **nxt)
-        else:
-            prog.gemm([act_seg(a1, cout, taps=9)], prog.const_bf16(name + ".w1", w1), cout, 9 * cout, B, Ho, Wo, cout,
-                      bias=prog.const_f32(name + ".b1", P(i, "Conv_1.bias")), resid=x0.t, alpha=INV_SQRT2,
-                      out_f32=out.t, stats=out.stats, **nxt)
-        if tape is not None:
-            tape.append(dict(kind="res", i=i, kw=kw, x0=x0, x1=x1, h=h, out=out, shortcut=shortcut, Ho=Ho, Wo=Wo))
-        return out
+        skip = pair(i, "Conv_2.weight", "Conv_2.bias") if cin != cout or mode != 0 else None
+        blk = ResBlock(f"m{i}", cin, cout, gn0=pair(i, "GroupNorm_0.weight", "GroupNorm_0.bias"),
+                       conv0=pair(i, "Conv_0.weight", "Conv_0.bias"), gn1=pair(i, "GroupNorm_1.weight", "GroupNorm_1.bias"),
+                       conv1=pair(i, "Conv_1.weight", "Conv_1.bias"), skip=skip, temb=view(temb_all, temb_off[i]),
+                       temb_ld=temb_ld, film=False, groups0=_groups(cin), groups1=_groups(cout), eps=EPS,
+                       alpha=INV_SQRT2, resample=mode)
+        return lower_resblock(prog, blk, B, x0, x1, fuse_gn1=fuse, next_gn=consumer_gn(i + 1, cout), tape=tape)
 
-    def attnblock(i, kw, x: Act):
-        """AttnBlockpp.forward, layerspp.py:75-91 (single head of width C, scale C^-1/2, skip_rescale)."""
-        C, H, W = x.C, x.H, x.W
-        T = H * W
-        name = f"m{i}"
-        if x.pre is not None:
-            hn = x.pre                    # GroupNorm_0 of this block came out of the producer's epilogue
-        else:
-            hn = prog.tensor(name + ".hn", B * T * C, "bf16")
-            prog.gn_apply(src0=x.t, stats0=x.stats, C0=C, P0=x.P,
-                          gamma=prog.const_f32(name + ".gn.w", P(i, "GroupNorm_0.weight")),
-                          beta=prog.const_f32(name + ".gn.b", P(i, "GroupNorm_0.bias")),
-                          B=B, H=H, W=W, groups=_groups(C), eps=1e-6, silu=0, out_bf16=hn)
-        wq, wk, wv = (P(i, f"NIN_{j}.W").t().contiguous() for j in range(3))   # NIN: y = x.W + b, W is [in, out]
-        bq, bk, bv = (P(i, f"NIN_{j}.b") for j in range(3))
-        if fuse_attn and tape is None and T == 256 and C == 256:
-            # the whole block behind the GroupNorm as one kernel (dp_attn.cu): q, k, v^T, the logits, P and o stay on chip
-            out = new_act(prog, name + ".out", B, C, H, W)
-            w3, b3 = P(i, "NIN_3.W").t().contiguous(), P(i, "NIN_3.b")
-            prog.attn_block(hn, prog.const_bf16(name + ".wqkv3", torch.cat([wq, wk, wv, w3], 0)),
-                            prog.const_f32(name + ".bqkv3", torch.cat([bq, bk, bv, b3])), x.t, out.t, out.stats,
-                            B, T, C, C ** -0.5, INV_SQRT2)
-            return out
-        o = prog.tensor(name + ".o", B * T * C, "bf16")
-        if T <= 64:
-            qkv = prog.tensor(name + ".qkv", B * T * 3 * C, "bf16")
-            prog.gemm([act_seg(hn, C)], prog.const_bf16(name + ".wqkv", torch.cat([wq, wk, wv], 0)),
-                      3 * C, C, 1, 1, B * T, 3 * C, bias=prog.const_f32(name + ".bqkv", torch.cat([bq, bk, bv])),
-                      out_bf16=qkv)
-            prog.attn_small(qkv, o, B, T, 1, C, C ** -0.5)
-        else:
-            assert T in (128, 256), "tensor-core attention path needs T in {128, 256}"
-            qk = prog.tensor(name + ".qk", B * T * 2 * C, "bf16")
-            prog.gemm([act_seg(hn, C)], prog.const_bf16(name + ".wqk", torch.cat([wq, wk], 0)), 2 * C, C, 1, 1,
-                      B * T, 2 * C, bias=prog.const_f32(name + ".bqk", torch.cat([bq, bk])), out_bf16=qk)
-            # V^T per sample: [C, T] = Wv[C, C] . hn_b[T, C]^T   (weights as the A operand, bias along M)
-            vt = prog.tensor(name + ".vt", B * C * T, "bf16")
-            prog.gemm([act_seg(prog.const_bf16(name + ".wv", wv), C)], hn, B * T, C, 1, 1, C, T, batch=B,
-                      a_batch_rows=0, b_batch_rows=T, out_batch_stride=C * T,
-                      bias=prog.const_f32(name + ".bv", bv), bias_along_m=1, out_bf16=vt, ldc=T)
-            # P = exp(scale * (q.k^T - rowmax)) (bf16) and its row sums
-            pm = prog.tensor(name + ".p", B * T * T, "bf16")
-            rs = prog.tensor(name + ".rowsum", B * T, "f32")
-            prog.gemm([act_seg(qk, C, c_total=2 * C)], view(qk, C), B * T, 2 * C, 1, 1, T, T, batch=B,
-                      a_batch_rows=T, b_batch_rows=T, out_batch_stride=T * T, out_bf16=pm, ldc=T, softmax=1,
-                      softmax_scale=C ** -0.5, rowsum_out=rs)
-            prog.gemm([act_seg(pm, T)], vt, B * C, T, 1, 1, T, C, batch=B, a_batch_rows=T, b_batch_rows=C,
-                      out_batch_stride=T * C, rowscale=rs, out_bf16=o, ldc=C)
-        out = new_act(prog, name + ".out", B, C, H, W)
-        nxt = gn_epilogue_args(out, consumer_gn(i + 1, C), name)
-        prog.gemm([act_seg(o, C)], prog.const_bf16(name + ".w3", P(i, "NIN_3.W").t().contiguous()), C, C, B, H, W, C,
-                  bias=prog.const_f32(name + ".b3", P(i, "NIN_3.b")), resid=x.t, alpha=INV_SQRT2, out_f32=out.t,
-                  stats=out.stats, **nxt)
-        if tape is not None:
-            rec = dict(kind="attn", i=i, x=x, out=out, T=T, C=C, scale=C ** -0.5)
-            if T <= 64:
-                rec.update(qkv=qkv)
-            else:
-                rec.update(qk=qk, vt=vt, pm=pm, rs=rs)
-            tape.append(rec)
-        return out
+    def attnblock(i, x: Act):
+        """AttnBlockpp.forward, layerspp.py:75-91 (single head of width C, scale C^-1/2, skip_rescale).
+        NIN: y = x.W + b with W [in, out]."""
+        q, k, v, o = ((P(i, f"NIN_{j}.W").t().contiguous(), P(i, f"NIN_{j}.b")) for j in range(4))
+        blk = AttnBlock(f"m{i}", pair(i, "GroupNorm_0.weight", "GroupNorm_0.bias"), q, k, v, o, heads=1,
+                        scale=x.C ** -0.5, groups=_groups(x.C), eps=EPS, alpha=INV_SQRT2)
+        # the whole block behind the GroupNorm as one kernel (dp_attn.cu): q, k, v^T, the logits, P and o stay on chip
+        one_kernel = fuse_attn and x.H * x.W == 256 and x.C == 256
+        return lower_attn_block(prog, blk, B, x, one_kernel=one_kernel,
+                                next_gn=None if one_kernel else consumer_gn(i + 1, x.C), tape=tape)
 
     # ---- walk the module list exactly as NCSNpp.forward does (ncsnpp.py:263-381) ----------------------
-    idx = 2
-    h0 = new_act(prog, "conv_in.out", B, nf, S, S)
-    prog.conv_in_gemm("conv_in", P(2, "weight"), P(2, "bias"), h0.t, h0.stats, B, S, S, nf)
+    h0 = lower_input_conv(prog, pair(2, "weight", "bias"), B, tape)
     idx = 3
     hs = [h0]
     nres = len(cfg.ch_mult)
     for lvl in range(nres):
         for _ in range(cfg.num_res_blocks):
-            kind, kw = plan[idx]
-            h = resblock(idx, kw, hs[-1])
+            h = resblock(idx, hs[-1])
             idx += 1
             if h.H in cfg.attn_resolutions:
-                h = attnblock(idx, plan[idx][1], h)
+                h = attnblock(idx, h)
                 idx += 1
             hs.append(h)
         if lvl != nres - 1:
-            hs.append(resblock(idx, plan[idx][1], hs[-1]))
+            hs.append(resblock(idx, hs[-1]))
             idx += 1
     h = hs[-1]
-    h = resblock(idx, plan[idx][1], h); idx += 1
-    h = attnblock(idx, plan[idx][1], h); idx += 1
-    h = resblock(idx, plan[idx][1], h); idx += 1
+    h = resblock(idx, h); idx += 1
+    h = attnblock(idx, h); idx += 1
+    h = resblock(idx, h); idx += 1
     for lvl in reversed(range(nres)):
         for _ in range(cfg.num_res_blocks + 1):
-            h = resblock(idx, plan[idx][1], h, hs.pop())
+            h = resblock(idx, h, hs.pop())
             idx += 1
         if h.H in cfg.attn_resolutions:
-            h = attnblock(idx, plan[idx][1], h)
+            h = attnblock(idx, h)
             idx += 1
         if lvl != 0:
-            h = resblock(idx, plan[idx][1], h)
+            h = resblock(idx, h)
             idx += 1
-    assert not hs
-    C = h.C
-    if tape is not None:
-        tape.append(dict(kind="gn_out", idx=idx, x=h))
-        tape.insert(0, dict(kind="conv_in", out=h0))
-        prog.meta.update(model="ncsnpp", out_channels=cfg.num_channels, cond="999*t")
-        return prog
-    if h.pre is not None:
-        a = h.pre                         # the output GroupNorm + act came out of the last block's epilogue
-    else:
-        a = prog.tensor("out.a", B * S * S * C, "bf16")
-        prog.gn_apply(src0=h.t, stats0=h.stats, C0=C, P0=h.P, gamma=prog.const_f32("out.gn.w", P(idx, "weight")),
-                      beta=prog.const_f32("out.gn.b", P(idx, "bias")), B=B, H=S, W=S, groups=_groups(C), eps=1e-6,
-                      silu=1, out_bf16=a)
-    idx += 1
-    prog.conv_out_gemm("out", a, P(idx, "weight"), P(idx, "bias"), B, S, S, C, cfg.num_channels)
-    idx += 1
-    assert idx == len(plan)
+    assert not hs and idx + 2 == len(plan)
+    lower_output_head(prog, h, pair(idx, "weight", "bias"), _groups(h.C), EPS, pair(idx + 1, "weight", "bias"), B, tape)
     prog.meta.update(model="ncsnpp", out_channels=cfg.num_channels, cond="999*t")
     return prog
 
@@ -367,125 +218,9 @@ def lower(cfg, sd, B, h_bf16=True, tape=None, fuse_gn=True, fuse_attn=True):
 def lower_vjp(cfg, sd, B):
     """Forward (with a tape) followed by the data-gradient ops: the program of `dp_unet_vjp`, gx = J(x, t)^T g.
 
-    Mirrors oracle/ncsnpp_vjp.py (held to torch.autograd on the reference-identical forward): every conv / NIN contributes
-    the same tcgen05 implicit GEMM with flipped / transposed weights, GroupNorm(+SiLU, +resample, +concat) the two-pass
-    `gn_bwd` op, attention GEMMs + `softmax_bwd` + bf16 transposes (`attn_small_bwd` for T <= 64). The gradient stream is
-    fp32 (like the residual stream), GEMM operands bf16. The reference reaches this through torchsde's adjoint
-    (runners/diffpure_sde.py:233-239); here the runner differentiates the discrete Euler loop it actually runs."""
+    Mirrors oracle/ncsnpp_vjp.py (held to torch.autograd on the reference-identical forward). The reference reaches this
+    through torchsde's adjoint (runners/diffpure_sde.py:233-239); here the runner differentiates the discrete Euler loop
+    it actually runs."""
     tape = []
     prog = lower(cfg, sd, B, tape=tape)
-    S, nf, ncol = cfg.image_size, cfg.nf, cfg.num_channels
-
-    def P(i, name):
-        return sd[f"all_modules.{i}.{name}"].detach().float().cpu()
-
-    grad = {}        # tensor index -> (fp32 gradient, bf16 copy) of a residual-stream tensor
-    skip_grad = {}   # tensor index -> fp32 gradient that reached the tensor through its skip connection
-
-    def gpair(name, n):
-        return prog.tensor(name + ".g32", n, "f32"), prog.tensor(name + ".g16", n, "bf16")
-
-    # ---- output conv + output GroupNorm -------------------------------------------------------------------
-    rec = tape[-1]
-    hl, idx = rec["x"], rec["idx"]
-    C = hl.C
-    gin = prog.tensor("bwd.gin", B * S * S * 64, "bf16")
-    prog.grad_in(gin, B, S, S, ncol, 64)
-    wout = torch.zeros(64, C, 3, 3)
-    wout[:ncol] = P(idx + 1, "weight")
-    ga = prog.tensor("bwd.out.ga", B * S * S * C, "f32")
-    prog.gemm([act_seg(gin, 64, taps=9)], prog.const_bf16("bwd.out.w", pack_dgrad3x3(wout)), C, 9 * 64, B, S, S, C,
-              out_f32=ga)
-    g32, g16 = gpair("bwd.out", B * S * S * C)
-    prog.gn_bwd(src0=hl.t, stats0=hl.stats, C0=C, P0=hl.P, gamma=prog.const_f32("bwd.out.gn.w", P(idx, "weight")),
-                beta=prog.const_f32("bwd.out.gn.b", P(idx, "bias")), B=B, H=S, W=S, groups=_groups(C), eps=1e-6, silu=1,
-                g=ga, d0_f32=g32, d0_bf16=g16)
-    grad[hl.t.index] = (g32, g16)
-
-    def res_bwd(r):
-        i, kw, x0, x1, h, Ho, Wo = r["i"], r["kw"], r["x0"], r["x1"], r["h"], r["Ho"], r["Wo"]
-        cin, cout, mode = kw["cin"], kw["cout"], kw["mode"]
-        H, W = x0.H, x0.W
-        name = f"bwd.m{i}"
-        g32, g16 = grad.pop(r["out"].t.index)
-        ga1 = prog.tensor(name + ".ga1", B * Ho * Wo * cout, "f32")
-        prog.gemm([act_seg(g16, cout, taps=9)], prog.const_bf16(name + ".w1", pack_dgrad3x3(P(i, "Conv_1.weight"))),
-                  cout, 9 * cout, B, Ho, Wo, cout, alpha=INV_SQRT2, out_f32=ga1)
-        gc0 = prog.tensor(name + ".gc0", B * Ho * Wo * cout, "bf16")
-        prog.gn_bwd(src0=h.t, stats0=h.stats, C0=cout, P0=h.P,
-                    gamma=prog.const_f32(name + ".gn1.w", P(i, "GroupNorm_1.weight")),
-                    beta=prog.const_f32(name + ".gn1.b", P(i, "GroupNorm_1.bias")), B=B, H=Ho, W=Wo,
-                    groups=_groups(cout), eps=1e-6, silu=1, g=ga1, d0_bf16=gc0)
-        ga0 = prog.tensor(name + ".ga0", B * Ho * Wo * cin, "f32")
-        prog.gemm([act_seg(gc0, cout, taps=9)], prog.const_bf16(name + ".w0", pack_dgrad3x3(P(i, "Conv_0.weight"))),
-                  cin, 9 * cout, B, Ho, Wo, cin, out_f32=ga0)
-        if r["shortcut"]:
-            gxs = prog.tensor(name + ".gxs", B * Ho * Wo * cin, "f32")
-            prog.gemm([act_seg(g16, cout)], prog.const_bf16(name + ".w2", pack_conv1x1(P(i, "Conv_2.weight")).t().contiguous()),
-                      cin, cout, B, Ho, Wo, cin, alpha=INV_SQRT2, out_f32=gxs)
-            add0, scale = gxs, 1.0
-        else:
-            add0, scale = g32, INV_SQRT2
-        d32, d16 = gpair(name + ".dx", B * H * W * x0.C)
-        d1 = prog.tensor(name + ".dskip", B * H * W * x1.C, "f32") if x1 else None
-        prog.gn_bwd(src0=x0.t, stats0=x0.stats, C0=x0.C, P0=x0.P, src1=x1.t if x1 else None,
-                    stats1=x1.stats if x1 else None, C1=x1.C if x1 else 0, P1=x1.P if x1 else 0,
-                    gamma=prog.const_f32(name + ".gn0.w", P(i, "GroupNorm_0.weight")),
-                    beta=prog.const_f32(name + ".gn0.b", P(i, "GroupNorm_0.bias")), B=B, H=H, W=W, groups=_groups(cin),
-                    eps=1e-6, silu=1, resample=mode, g=ga0, add0=add0, add0_scale=scale,
-                    add1=skip_grad.pop(x0.t.index, None), d0_f32=d32, d0_bf16=d16, d1_f32=d1)
-        grad[x0.t.index] = (d32, d16)
-        if x1:
-            skip_grad[x1.t.index] = d1
-
-    def attn_bwd(r):
-        i, x, T, C, scale = r["i"], r["x"], r["T"], r["C"], r["scale"]
-        H, W = x.H, x.W
-        name = f"bwd.m{i}"
-        g32, g16 = grad.pop(r["out"].t.index)
-        go = prog.tensor(name + ".go", B * T * C, "bf16")
-        prog.gemm([act_seg(g16, C)], prog.const_bf16(name + ".w3", P(i, "NIN_3.W").contiguous()), C, C, 1, 1, B * T, C,
-                  alpha=INV_SQRT2, out_bf16=go)
-        dqkv = prog.tensor(name + ".dqkv", B * T * 3 * C, "bf16")
-        if T <= 64:
-            prog.attn_small_bwd(r["qkv"], go, dqkv, B, T, 1, C, scale)
-        else:
-            qk, vt, pm, rs = r["qk"], r["vt"], r["pm"], r["rs"]
-            tr = lambda nm, src, rows, cols, ld_in, ibs: _transposed(prog, name + nm, src, rows, cols, ld_in, ibs, B)  # noqa: E731
-            v = tr(".v", vt, C, T, T, C * T)                     # [B][T][C]
-            qT = tr(".qT", view(qk, 0), T, C, 2 * C, T * 2 * C)    # [B][C][T]
-            kT = tr(".kT", view(qk, C), T, C, 2 * C, T * 2 * C)
-            goT = tr(".goT", go, T, C, C, T * C)
-            dp = prog.tensor(name + ".dp", B * T * T, "f32")
-            prog.gemm([act_seg(go, C)], v, B * T, C, 1, 1, T, T, batch=B, a_batch_rows=T, b_batch_rows=T,
-                      out_batch_stride=T * T, out_f32=dp, ldc=T)
-            ds = prog.tensor(name + ".ds", B * T * T, "bf16")
-            pn = prog.tensor(name + ".pn", B * T * T, "bf16")
-            prog.softmax_bwd(pm, rs, dp, ds, pn, B * T, T)
-            dsT = tr(".dsT", ds, T, T, T, T * T)
-            pnT = tr(".pnT", pn, T, T, T, T * T)
-            bat = dict(batch=B, a_batch_rows=T, b_batch_rows=C, out_batch_stride=T * 3 * C, ldc=3 * C)
-            prog.gemm([act_seg(ds, T)], kT, B * C, T, 1, 1, T, C, alpha=scale, out_bf16=view(dqkv, 0), **bat)
-            prog.gemm([act_seg(dsT, T)], qT, B * C, T, 1, 1, T, C, alpha=scale, out_bf16=view(dqkv, C), **bat)
-            prog.gemm([act_seg(pnT, T)], goT, B * C, T, 1, 1, T, C, out_bf16=view(dqkv, 2 * C), **bat)
-        ghn = prog.tensor(name + ".ghn", B * T * C, "f32")
-        wqkv = torch.cat([P(i, f"NIN_{j}.W") for j in range(3)], dim=1).contiguous()      # [C_in, 3 C_out]
-        prog.gemm([act_seg(dqkv, 3 * C)], prog.const_bf16(name + ".wqkv", wqkv), C, 3 * C, 1, 1, B * T, C, out_f32=ghn)
-        d32, d16 = gpair(name + ".dx", B * T * C)
-        prog.gn_bwd(src0=x.t, stats0=x.stats, C0=C, P0=x.P, gamma=prog.const_f32(name + ".gn.w", P(i, "GroupNorm_0.weight")),
-                    beta=prog.const_f32(name + ".gn.b", P(i, "GroupNorm_0.bias")), B=B, H=H, W=W, groups=_groups(C),
-                    eps=1e-6, silu=0, g=ghn, add0=g32, add0_scale=INV_SQRT2, add1=skip_grad.pop(x.t.index, None),
-                    d0_f32=d32, d0_bf16=d16)
-        grad[x.t.index] = (d32, d16)
-
-    for r in reversed(tape[1:-1]):
-        (res_bwd if r["kind"] == "res" else attn_bwd)(r)
-    h0 = tape[0]["out"]
-    _, g16 = grad.pop(h0.t.index)
-    assert not grad and not skip_grad, (list(grad), list(skip_grad))
-    gx8 = prog.tensor("bwd.gx8", B * S * S * 8, "f32")
-    prog.gemm([act_seg(g16, nf, taps=9)], prog.const_bf16("bwd.conv_in.w", pack_dgrad3x3(P(2, "weight"))), ncol, 9 * nf,
-              B, S, S, 8, out_f32=gx8, ldc=8)
-    prog.update(gx8, 8, B, S, S, ncol)
-    prog.meta.update(vjp=True)
-    return prog
+    return lower_data_gradient(prog, tape, B, g_channels=cfg.num_channels)
